@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- CycleGAN-VC training-step throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16x3|bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16x3|bf16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one synthetic minibatch: G_A2B/G_B2A/D_A/D_B forward + cycle/identity/
@@ -12,6 +12,16 @@ Prints ONE JSON line (rank 0).  `value` is 256-sample steps per second summed ov
 on device-resident inputs; `e2e` is the same through CycleGAN.train() with host buffers (H2D of A and B and D2H of
 the losses inside the timed region).  `--impl reference` times the CPU oracle (a torch-CPU restatement of the
 reference graph; TensorFlow 1.x cannot be installed here -- see DESIGN.md) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step computed, as float32 `.npy` files, so that two builds can be compared
+output for output (inputs and initial weights are seeded, so the same arguments give the same inputs in every run):
+  train: losses.npy (the 8 losses, cgvc.native.LOSS_NAMES order) and params_sample.npy (the updated weights at DUMP_SAMPLE
+         positions of the parameters concatenated in CycleGAN.param_names() order, drawn without replacement with seed 0, ascending);
+  infer: converted_A2B.npy (the whole [1024, 24, 128] generator output).
+The generator forward is deterministic: two runs of one build give bit-identical infer dumps.  A train step is not (the order of
+its gradient atomics varies, and Adam's sign-descent early steps amplify that), so two runs of one build differ too: measured
+after 3 warm-up + 10 timed default steps on a B200 at a 1000 W power limit, 7e-4 relative L2 on losses.npy and 5e-3 on
+params_sample.npy.  Compare train dumps of two builds against that spread, not for equality.
 """
 from __future__ import annotations
 
@@ -27,6 +37,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 BATCH = 256
 FRAMES = 128
@@ -37,6 +48,17 @@ GFLOP_EXECUTED_PER_SAMPLE_STEP = 85.96                          # what the engin
 GFLOP_GENERATOR_FWD = 2.656043                                  # one generator application per sample (T = 128)
 METRIC = "CycleGAN-VC train steps/sec @ batch 256x[24,128] MCEP"
 UNIT = "steps/s (256-sample steps, summed over GPUs)"
+DUMP_SAMPLE = 1 << 22                                           # weights in params_sample.npy (16 MB of the 479 MB)
+
+
+def dump_train_outputs(m, losses, out_dir):
+    """--dump-outputs of the train workload: the last step's losses and a fixed sample of the weights it left."""
+    import numpy as np
+    flat = np.concatenate([p.ravel() for p in m.get_params().values()])
+    pick = np.sort(np.random.default_rng(0).choice(flat.size, DUMP_SAMPLE, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "losses.npy"), np.asarray(losses, dtype=np.float32))
+    np.save(os.path.join(out_dir, "params_sample.npy"), flat[pick])
 
 
 def _peaks():
@@ -213,16 +235,18 @@ def pick_reference_batch(steps, warmup, budget_s, threads):
     return 16, per_sample
 
 
-def infer_measure(precision, local_rank, world, dist, steps, warmup):
+def infer_measure(precision, local_rank, world, dist, steps, warmup, dump_dir=None):
     """BASELINE.json configs[4] (convert.py path): generator-only A2B forward of 1024 x [24,128] per GPU.  Embarrassingly parallel
-    over GPUs (no collective).  Returns a dict (rank 0) with frames/s device-resident and end to end (host numpy in / out)."""
+    over GPUs (no collective).  Returns a dict (rank 0) with frames/s device-resident and end to end (host numpy in / out).
+    With `dump_dir`, the output of the last timed forward goes to dump_dir/converted_A2B.npy."""
     import numpy as np
     import torch
     import cgvc
     dev = torch.device("cuda", local_rank)
     nb = 1024
     m = cgvc.CycleGAN(num_features=FEATS, mode="test", max_batch=nb, max_frames=FRAMES, precision=precision, device=local_rank, seed=0)
-    x = torch.randn(nb, FEATS, FRAMES, device=dev)
+    g = torch.Generator(device=dev); g.manual_seed(2000)
+    x = torch.randn(nb, FEATS, FRAMES, device=dev, generator=g)
     for _ in range(max(warmup, 3)):
         m.test(x, "A2B")
     if dist is not None:
@@ -231,9 +255,12 @@ def infer_measure(precision, local_rank, world, dist, steps, warmup):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        m.test(x, "A2B")
+        y = m.test(x, "A2B")
     e1.record(); torch.cuda.synchronize(dev)
     ms = e0.elapsed_time(e1)
+    if dump_dir is not None:
+        os.makedirs(dump_dir, exist_ok=True)
+        np.save(os.path.join(dump_dir, "converted_A2B.npy"), y.cpu().numpy())
     # end to end: host float32 utterance crops in, converted host array out (pinned staging, H2D + D2H inside the timed region)
     xh = x.cpu().numpy()
     m.test(xh, "A2B")
@@ -271,7 +298,7 @@ def infer_bench(args, rank, local_rank, world):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    r = infer_measure(args.precision, local_rank, world, dist, args.steps, args.warmup)
+    r = infer_measure(args.precision, local_rank, world, dist, args.steps, args.warmup, dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
     if rank == 0:
         r.update({"warmup": max(args.warmup, 3), "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "data": "synthetic", "clocks": clocks,
@@ -307,14 +334,20 @@ def main():
                     help="engine option (include/cgvc.h: side_wgrad, cta_pairs, post_onepass, fuse_in, ...) for A/B measurements; repeatable")
     ap.add_argument("--workload", default="train", choices=["train", "infer"],
                     help="train: the headline metric; infer: BASELINE config 5, generator-only forward of 1024 x [24,128] (frames/s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/*.npy (float32; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs records the native engine's outputs (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1:
         mute_stdout()
-    steps, warmup = max(args.steps, 1), max(args.warmup, 3 if args.impl == "ours" else 0)
+    steps, warmup = args.steps, max(args.warmup, 3 if args.impl == "ours" else 0)
     workload = ("full CycleGAN-VC train step (4 generator + 2 discriminator applications fwd, losses, bwd, 2x Adam), "
                 "batch %d x [24 MCEP, 128 frames] per GPU, synthetic N(0,1) MCEP, glorot weights" % args.batch)
     config = {"workload": workload, "per_gpu_batch": args.batch, "frames": FRAMES, "parallelism": "dp%d" % max(world, 1), "precision": args.precision,
@@ -407,6 +440,8 @@ def main():
     ms_per_step = ms / steps
     value = world * (args.batch / BATCH) * steps / (ms / 1e3)
     losses = m._losses.cpu().numpy().tolist()
+    if args.dump_outputs is not None and rank == 0:
+        dump_train_outputs(m, losses, args.dump_outputs)            # before the untimed steps below move the weights on
 
     # ---- end to end through the reference-facing API: host numpy in, losses out, copies inside the timed region
     A_host = A.cpu().numpy().astype(np.float32); B_host = B.cpu().numpy().astype(np.float32)
