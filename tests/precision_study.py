@@ -27,13 +27,9 @@ import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from oracle import cyclegan_oracle as O  # noqa: E402
-
-F64 = torch.float64
-
-
-def rn(x, dt):
-    return x.to(dt).to(F64)
+from scheme_ref import F64, planes_bf16x3, planes_f16f8, rn  # noqa: E402  (the engine's plane definitions, stated once)
 
 
 def q_tf32(x):
@@ -70,16 +66,12 @@ LOSS_SCALE = 1.0      # fp16_f8_train: every upstream gradient is multiplied by 
 
 def _q_act(x):
     """activation-role planes: q16, e4m3(q16), e4m3(lo * 2^12) -> (hi16, hi8, lo8 already divided back)"""
-    h, l = split(x, torch.float16)
-    sat = lambda t: t.clamp(-448.0, 448.0)
-    return h, rn(sat(h), E4), rn(sat(l * 4096.0), E4) / 4096.0
+    return planes_f16f8(x, "act")
 
 
 def _q_w(x):
     """weight-role planes: q16, e4m3(q16 * 2^3), e4m3(lo * 2^15)"""
-    h, l = split(x, torch.float16)
-    sat = lambda t: t.clamp(-448.0, 448.0)
-    return h, rn(sat(h * 8.0), E4) / 8.0, rn(sat(l * 32768.0), E4) / 32768.0
+    return planes_f16f8(x, "weight")
 
 
 def terms(a, b, scheme, role="fwd"):
@@ -102,8 +94,7 @@ def terms(a, b, scheme, role="fwd"):
     if scheme == "tf32":
         return [(q_tf32(a), q_tf32(b))]
     if scheme == "bf16x3":                       # the engine's current mode: hi*hi + hi*lo + lo*hi, lo kept in bf16
-        ah, al = split(a, torch.bfloat16); bh, bl = split(b, torch.bfloat16)
-        al, bl = rn(al, torch.bfloat16), rn(bl, torch.bfloat16)
+        (ah, al), (bh, bl) = planes_bf16x3(a), planes_bf16x3(b)
         return [(ah, bh), (ah, bl), (al, bh)]
     if scheme == "fp16x2":                       # A exact to 22 bits, B rounded to fp16: (ah+al)*bh
         ah, al = split(a, torch.float16); bh = rn(b, torch.float16)
@@ -118,9 +109,9 @@ def terms(a, b, scheme, role="fwd"):
     if scheme == "fp16_f8_static":
         # the forward-pass variant sketched in DESIGN.md 10: STATIC power-of-two scales (no amax pass):
         #   a_hi8 = e4m3(a_hi), b_lo8 = e4m3(b_lo * 2^15);  a_lo8 = e4m3(a_lo * 2^12), b_hi8 = e4m3(b_hi * 2^3); both products * 2^-15
-        ah, al = split(a, torch.float16); bh, bl = split(b, torch.float16)
-        sat = lambda x: x.clamp(-448.0, 448.0)
-        return [(ah, bh), (rn(sat(ah), E4), rn(sat(bl * 2.0 ** 15), E4) * 2.0 ** -15), (rn(sat(al * 2.0 ** 12), E4) * 2.0 ** -12, rn(sat(bh * 8.0), E4) / 8.0)]
+        ah, ah8, al8 = _q_act(a)
+        bh, bh8, bl8 = _q_w(b)
+        return [(ah, bh), (ah8, bl8), (al8, bh8)]
     raise ValueError(scheme)
 
 
